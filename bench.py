@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W [--impl vcl|reference|library]
                     [--config 2|3|4|5] [--clips B] [--model 7b|13b] [--frames 32,64,100]
+                    [--dump-outputs DIR]
 
 Configurations (numbering of SURVEY.md 8d; BASELINE.json `configs` is 0-based, so config k = configs[k-1]):
   2  (default, the configuration the metric is quoted on) 1 clip per GPU: 100 synthetic 224x224
@@ -34,6 +35,11 @@ Printed JSON (rank 0, one line):
                        cost on the box (SURVEY.md 2.3); 1 warm-up + 1 timed clip
 `--impl reference` times the CPU path as the arm of its own (rank 0 only; one bounded sample whatever
 --steps says); `--impl library` prints the library baseline alone.
+
+`--dump-outputs DIR` (--impl vcl) writes what the last timed device-resident step returned, on rank 0, as
+DIR/<name>.npy in float32: `tokens` [clips, 32] (all ranks' clips with N GPUs) and `video_features`
+[clips, 356, 1024] (configs 2-4), or `video_features_T<t>` [356, 1024] per frame count (config 5). Weights
+and inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -60,6 +66,7 @@ CONFIGS = {2: dict(model="7b", clips=1, label="configs[1]: single clip, 100 fram
            5: dict(model="7b", clips=1, label="configs[4]: CLIP-only throughput sweep, 1000 clips x {32,64,100} frames")}
 METRIC = "videos/sec (100-frame CLIP encode + 7B 32-tok decode)"
 SWEEP_CLIPS = 1000
+DUMP_BYTES = 60 * 10 ** 6          # --dump-outputs: array data in all, under 64 MB with the .npy headers
 
 
 def peaks():
@@ -105,6 +112,22 @@ def workload_config(cfg_id, model, B, world):
             "weights": "random-init bf16 (seed 0)",
             "l2": "no flush: every step streams inputs+weights far larger than L2 "
                   f"({w['weights_step'] / 1e9:.1f} GB of weights per decode step vs 126 MB)"}
+
+
+def dump_outputs(path, arrays):
+    """Write {name: tensor} as path/<name>.npy in float32 (token ids below 2^24 stay exact). Smallest first,
+    an array larger than its share of what is left of DUMP_BYTES keeps a fixed, seeded subset of its
+    leading-axis rows, so a larger --clips still gives the same rows on every run."""
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_BYTES
+    for i, (name, t) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].numel())):
+        a = t.float().cpu().numpy()
+        share = left // (len(arrays) - i)
+        if a.nbytes > share:
+            keep = max(1, share * len(a) // a.nbytes)
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+        left -= a.nbytes
 
 
 def metric_name(cfg_id, model):
@@ -511,11 +534,15 @@ def run_vcl(args, rank, world, local_rank):
         clocks.start()
         ms_dev, evs = timed(args.steps, 4, False)
         launches = vn.launch_count() - l0
+        outputs = {"tokens": (gathered if gathered is not None else toks).clone(),
+                   "video_features": feats.clone()} if args.dump_outputs and rank == 0 else None
         ms_e2e, _ = timed(args.steps, 0, True)
         clk = clocks.stop()
         stream.synchronize()
         api_tokens = toks_h.clone()
         agree = bool(torch.equal(api_tokens, toks.cpu()))
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     stage = np.array([[ev[i].elapsed_time(ev[i + 1]) for i in range(3)] for ev in evs]).mean(0)  # ms: clip, prefill, decode
 
     w = work(args.model)
@@ -622,8 +649,11 @@ def run_clip_sweep(args, rank, world, local_rank):
         clocks.start()
         ms_dev, evs = timed(args.steps, len(Ts) + 1, False)
         launches = vn.launch_count() - l0
+        outputs = {f"video_features_T{t}": outs[t].clone() for t in Ts} if args.dump_outputs and rank == 0 else None
         ms_e2e, _ = timed(args.steps, 0, True)
         clk = clocks.stop()
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     per_t = np.array([[ev[i].elapsed_time(ev[i + 1]) for i in range(len(Ts))] for ev in evs]).mean(0)   # ms per clip at each T
     hbm, tf, src = peaks()
     sweep = {}
@@ -722,7 +752,13 @@ def main():
     ap.add_argument("--frames", default="32,64,100", help="config 5: frames per clip, comma separated")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-library", action="store_true", help="skip the library_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "vcl":
+        ap.error("--dump-outputs needs --impl vcl")
     if args.model is None:
         args.model = CONFIGS[args.config]["model"]
     if args.clips is None:

@@ -1,4 +1,5 @@
-"""Helpers shared by the GPU parity tests: build a vcl Engine from oracle configs."""
+"""Helpers shared by the tests: build a vcl Engine from oracle configs, load the golden fixtures."""
+import numpy as np
 import torch
 
 import vcl_native as vn
@@ -19,6 +20,16 @@ def make_engine(clip: O.ClipCfg | None = None, llm: O.LlmCfg | None = None, clip
     c.n_temporal = 100
     c.max_frames, c.max_batch, c.max_seq = max_frames, max_batch, max_seq
     return vn.Engine(c)
+
+
+def load_pool_golden(path):
+    """golden/pool.npz as a dict, with the reference's numpy-pooling results rebuilt from the stored XOR of
+    their fp16 bit patterns with the torch-pooling results (golden/make_golden.py)."""
+    g = dict(np.load(path))
+    for k in ("t8_numpy", "t100_numpy_rows"):
+        torch_bits = g[k.replace("numpy", "torch")].view(np.uint16)
+        g[k] = (torch_bits ^ g.pop(k + "_xor_torch")).view(np.float16)
+    return g
 
 
 def to_dev(sd, dtype=torch.bfloat16, device="cuda"):

@@ -1,14 +1,14 @@
 """Generate the golden fixtures in this directory by running THE REFERENCE ITSELF.
 
-Run in the build container only (it needs /root/reference, which does not exist on the GPU box):
+It needs a checkout of PG-Video-LLaVA (mbzuai-oryx/Video-LLaVA); the tests only read the fixtures:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>
 
 What is executed (nothing from this repo's product code, and no copy of reference source):
-  * /root/reference/video_chatgpt/model/video_chatgpt.py : VideoChatGPTLlamaForCausalLM.forward
+  * <reference>/video_chatgpt/model/video_chatgpt.py : VideoChatGPTLlamaForCausalLM.forward
     (embedding splice, mm_projector, lm_head) on top of the installed transformers LlamaModel
-  * /root/reference/video_chatgpt/inference.py : get_spatio_temporal_features_torch
-  * /root/reference/scripts/save_spatio_temporal_clip_features.py : get_spatio_temporal_features
+  * <reference>/video_chatgpt/inference.py : get_spatio_temporal_features_torch
+  * <reference>/scripts/save_spatio_temporal_clip_features.py : get_spatio_temporal_features
   * transformers.CLIPVisionModel (what the reference instantiates for its vision tower,
     video_chatgpt/eval/model_utils.py:134), attn_implementation="eager"
 all in fp32 on CPU, with the seeded synthetic weights/inputs of oracle/vcl_oracle.py
@@ -19,7 +19,9 @@ prepare_inputs_for_generation (video_chatgpt.py:253-257).
 
 Outputs (all small; see tests/test_oracle_cpu.py and tests/test_parity_gpu.py for their use):
   clip_tiny.npz   3-layer ViT (full width 1024), 3 frames: slices + row norms of hidden_states[0..2]
-  pool.npz        reference torch and numpy pooling of seeded fp16 features, T=8 (padded) and T=100
+  pool.npz        reference torch and numpy pooling of seeded fp16 features, T=8 (padded) and T=100;
+                  the numpy results are stored as the XOR of their fp16 bit patterns with the torch
+                  results (*_xor_torch), which keeps the file small (tests/_util.py: load_pool_golden)
   config1.npz     BASELINE config 1: 8 frames, full 24-layer ViT-L/14 -> pooled [356,1024] (fp32 run)
   llm_tiny.npz    2-layer LLaMA (hidden 512, 4 heads), B=2, S=448: last-row logits, hidden slices,
                   8 greedy tokens per clip; plus the malformed-span error behaviour
@@ -40,8 +42,11 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
+if len(sys.argv) != 2:
+    sys.exit("usage: python tests/golden/make_golden.py <reference checkout>")
+REF = os.path.abspath(sys.argv[1])
 sys.path.insert(0, ROOT)
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, REF)
 
 # the reference imports decord at module import time (eval/model_utils.py:4); it is not installed
 sys.modules.setdefault("decord", types.SimpleNamespace(VideoReader=None, cpu=None))
@@ -54,7 +59,7 @@ from video_chatgpt.model.video_chatgpt import (VideoChatGPTConfig,  # noqa: E402
                                                VideoChatGPTLlamaForCausalLM)
 
 _spec = importlib.util.spec_from_file_location(
-    "ref_save_features", "/root/reference/scripts/save_spatio_temporal_clip_features.py")
+    "ref_save_features", os.path.join(REF, "scripts", "save_spatio_temporal_clip_features.py"))
 
 
 def _load_ref_numpy_pool():
@@ -151,8 +156,13 @@ def main():
         # bf16 input (what the bf16 benchmark model feeds), as the reference function handles it
         "t100_bf16_rows": get_spatio_temporal_features_torch(f100.bfloat16()).numpy()[::7],
     }
-    np.savez_compressed(os.path.join(HERE, "pool.npz"), **pool)
     print("pool:", {k: (v.shape, v.dtype) for k, v in pool.items()})
+    # the two reference variants agree in (nearly) every bit: stored as bit differences they compress to
+    # almost nothing, where a second full copy would double the file
+    for k in ("t8_numpy", "t100_numpy_rows"):
+        torch_k = k.replace("numpy", "torch")
+        pool[k + "_xor_torch"] = pool.pop(k).view(np.uint16) ^ pool[torch_k].view(np.uint16)
+    np.savez_compressed(os.path.join(HERE, "pool.npz"), **pool)
 
     # ---------------- config 1 (BASELINE.json configs[0]) ----------------
     fcfg = O.ClipCfg()

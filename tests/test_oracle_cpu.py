@@ -37,7 +37,8 @@ def test_clip_tiny_matches_hf_reference():
 
 
 def test_pool_torch_and_numpy_bit_exact():
-    g = _load("pool.npz")
+    from _util import load_pool_golden
+    g = load_pool_golden(os.path.join(G, "pool.npz"))
     gen = torch.Generator().manual_seed(5)
     f8 = torch.randn(8, 256, 1024, generator=gen).half()
     f100 = torch.randn(100, 256, 1024, generator=gen).half()
