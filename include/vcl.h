@@ -173,6 +173,50 @@ int vcl_llm_generate(vcl_handle* h, const int64_t* ids, const void* video_feats,
 int vcl_llm_decode_loop(vcl_handle* h, const int32_t* first_tok, int B, int S, int n_new,
                         int32_t* out_tokens, void* stream);
 
+/* ---- sampling (do_sample=True): temperature -> top-k -> softmax -> multinomial on the device ----
+ * The reference's callers sample (inference.py:105-112: do_sample=True, temperature=0.2, HF's default
+ * top-k 50). HF applies TemperatureLogitsWarper, TopKLogitsWarper ($TF/generation/logits_process.py),
+ * softmax and torch.multinomial; the contract here, for row b and the fp32 logits l[0..V) the logits
+ * kernels write (bf16-rounded values), is:
+ *   - temperature <= 0: the arg-max, lowest index winning (the token vcl_llm_generate would produce);
+ *   - k = top_k if 1 <= top_k < V, else V (0: no filter); tau = the k-th largest logit counting
+ *     multiplicity; the kept set is K = {i : l_i >= tau} (every tie at tau stays, so |K| can exceed k);
+ *     NaN counts as -inf;
+ *   - weights w_i = exp(((double)l_i - (double)max l) / (double)T) in fp64 (HF's softmax is fp32: the
+ *     probabilities differ by ~1e-7 relative, in exchange for an exact host restatement);
+ *   - u in [0,1), t = u * sum_K w_i; the token is the smallest id of K, walking ids in ascending order,
+ *     whose running sum exceeds t (the largest id of K if rounding leaves none). The device sums in a
+ *     different association than a sequential walk, so a draw within ~1e-16 Z of a bin edge may land on the
+ *     neighbouring id;
+ *   - u = (w0 >> 11) * 2^-53, w0 = word 0 of Philox4x64-10 with key (seed, 0) at counter (pos, b, 0, 0),
+ *     pos = the sequence position the sampled token will occupy (the first new token after an S-token
+ *     prompt is at S), b = the row within the call. The stream therefore does not depend on chunking,
+ *     graph or eager launches, or the decode kernel family. (numpy.random.Philox(key=[seed, 0],
+ *     counter=[pos - 1, b, 0, 0]).random_raw(4)[0] is the same word: numpy increments before generating.)
+ * A row without a finite maximum yields the lowest id at its maximum (id 0 when every logit is -inf or NaN).
+ * vcl_sampling is a HOST struct, read when the call is made. */
+typedef struct vcl_sampling {
+  float temperature;
+  int32_t top_k;
+  uint64_t seed;
+} vcl_sampling;
+
+/* vcl_llm_generate with sampling: prefill, the first token sampled at position S, n_new-1 sampled decode
+ * steps from a CUDA graph kept per (B, n_new, mode) under the same LRU bound (one sampled graph serves every
+ * temperature, top-k, seed and prompt length). Sampled steps hand full logits to the sampler, so there is
+ * no partial arg-max hand-off on this path. */
+int vcl_llm_generate_sampled(vcl_handle* h, const int64_t* ids, const void* video_feats, const int32_t* vid_start,
+                             int B, int S, int n_new, const vcl_sampling* sampling, int32_t* out_tokens,
+                             void* stream);
+/* vcl_llm_decode_loop with sampling: first_tok [B] is the token at position S; token i of the output takes
+ * position S + i. */
+int vcl_llm_decode_loop_sampled(vcl_handle* h, const int32_t* first_tok, int B, int S, int n_new,
+                                const vcl_sampling* sampling, int32_t* out_tokens, void* stream);
+/* tok_out[b] = the token sampled from logits row b (fp32, row pitch ld elements, V columns) for sequence
+ * position pos (row b uses counter (pos, b)): the first token after vcl_llm_prefill_append, and the tests. */
+int vcl_op_sample(const float* logits, int64_t ld, int B, int V, const vcl_sampling* sampling, int pos,
+                  int32_t* tok_out, void* stream);
+
 /* Number of kernels of this library launched so far in the process (CUDA-graph replays count the
  * kernel nodes they contain). Evidence for bench.py's "gpu_launches". */
 long long vcl_launch_count(void);

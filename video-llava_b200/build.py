@@ -17,7 +17,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libvcl.so")
-SOURCES = ["vcl_api.cu", "gemm_tc.cu", "gemv.cu", "gemv_tc.cu", "gemv_tcw.cu", "gemv_mma.cu", "attention.cu", "attention_tc.cu", "attention_prefill_tc.cu", "decode_attention.cu", "elementwise.cu", "st_pool.cu"]
+SOURCES = ["vcl_api.cu", "gemm_tc.cu", "gemv.cu", "gemv_tc.cu", "gemv_tcw.cu", "gemv_mma.cu", "attention.cu", "attention_tc.cu", "attention_prefill_tc.cu", "decode_attention.cu", "elementwise.cu", "st_pool.cu", "sample.cu"]
 HEADERS = ["common.cuh", "kernels.h", os.path.join("..", "..", "include", "vcl.h")]
 
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]

@@ -80,6 +80,15 @@ int launch_argmax(const float* logits, int* out, long long out_stride, int B, in
                   cudaStream_t stream);
 int launch_set_int(int* dst, int value, cudaStream_t stream);
 
+// ---- sample.cu : temperature / top-k sampling, the contract of vcl_sampling (include/vcl.h) ----------
+struct SampleParams { float temperature; int top_k; unsigned long long seed; };   // layout of vcl_sampling
+// out[b * out_stride] = the token sampled from row b of logits (pitch ld) for sequence position
+// pos (+ *pos_dev); the parameters are read from params_dev when it is non-null, else taken from params
+int launch_sample(const float* logits, long long ld, int B, int V, const SampleParams* params_dev,
+                  const SampleParams& params, int pos, const int* pos_dev, int* out, long long out_stride,
+                  cudaStream_t stream);
+int launch_set_sample_params(SampleParams* dst, const SampleParams& p, cudaStream_t stream);
+
 // ---- st_pool.cu ---------------------------------------------------------------------------------
 // dtype codes: 0 = fp16, 1 = bf16
 int launch_st_pool(const void* feats, int in_dtype, long long frame_stride, long long patch_stride,

@@ -7,6 +7,7 @@
 // compute path and never touches a CPU implementation.
 #include "../../include/vcl.h"
 
+#include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -48,8 +49,10 @@ struct LlmLayerW {
   bf16 *ln1, *wqkv, *wo, *ln2, *wgu, *wd;
   bf16 *wqkv_t = nullptr, *wo_t = nullptr, *wgu_t = nullptr, *wd_t = nullptr;   // tiled copies for B = 1 decode
 };
+enum DecodeMode { MODE_GREEDY = 0, MODE_SAMPLED = 1 };
 struct GraphEntry {
   int B, S, n_new;     // S = -1: the prompt length is read on the device (h->d_pos), any S replays it
+  int mode;            // DecodeMode; a sampled graph reads its parameters from h->d_sample
   cudaGraphExec_t exec;
   long long kernels;   // kernel nodes in the graph (for vcl_launch_count)
   unsigned long long last_use;
@@ -65,6 +68,7 @@ struct StepIo {
   float* logits_out = nullptr;
   int32_t* tok_out = nullptr; long long out_stride = 1;
   const int* pos_dev = nullptr;   // position = pos + *pos_dev
+  bool sample = false;            // tok_out is sampled with the parameters in h->d_sample instead of the arg-max
 };
 
 }  // namespace
@@ -98,6 +102,7 @@ struct vcl_handle {
   std::vector<GraphEntry> graphs;
   unsigned long long graph_clock = 0;
   int* d_pos = nullptr;                        // prompt length of the running decode loop (device scalar)
+  SampleParams* d_sample = nullptr;            // sampling parameters of the running sampled loop
   ArgmaxPart* amax = nullptr;                  // [#SMs][max_batch] per-CTA partial arg-max of the logits kernel
   bool force_legacy_attention = false;
 
@@ -245,6 +250,7 @@ int vcl_create(vcl_handle** out, const vcl_config* c) {
   rc |= dalloc(h, &h->d_attn, xwin_elems((int)Bm, (int)D) > Bm * D ? xwin_elems((int)Bm, (int)D) : Bm * D);
   rc |= dalloc(h, &h->d_act, xwin_elems((int)Bm, (int)LF) > Bm * LF ? xwin_elems((int)Bm, (int)LF) : Bm * LF);
   rc |= dalloc(h, &h->d_pos, 4);
+  rc |= dalloc(h, &h->d_sample, 1);
   rc |= dalloc(h, &h->amax, (size_t)device_num_sms() * Bm);
   if (rc == 0) rc = launch_rope_table(h->rope_cos, h->rope_sin, c->max_seq, 128, c->rope_theta, 0);
   if (rc == 0) {
@@ -469,8 +475,10 @@ static bool tc_batch(vcl_handle* h, int B) {
 
 // final RMSNorm + lm_head on rows x[b*ldx .. ] (b < B), arg-max
 // partials_out: the arg-max is left as per-CTA partials in h->amax for the next step's q|k|v kernel
+// sample_pos >= 0: tok_out is sampled (parameters in h->d_sample) for sequence position sample_pos (+ *pos_dev)
 int lm_head_argmax(vcl_handle* h, const bf16* x, long long ldx, int B, float* logits_out,
-                   int32_t* tok_out, long long tok_stride, cudaStream_t st, bool partials_out = false) {
+                   int32_t* tok_out, long long tok_stride, cudaStream_t st, bool partials_out = false,
+                   int sample_pos = -1, const int* pos_dev = nullptr) {
   const vcl_config& c = h->cfg;
   if (partials_out) {
     GemvArgs g;
@@ -504,7 +512,13 @@ int lm_head_argmax(vcl_handle* h, const bf16* x, long long ldx, int B, float* lo
   if (logits_out != nullptr && logits_out != h->logits)
     VCL_CUDA_OK(cudaMemcpyAsync(logits_out, h->logits, (size_t)B * c.vocab * sizeof(float),
                                 cudaMemcpyDeviceToDevice, st));
-  if (tok_out != nullptr) VCL_TRY(launch_argmax(h->logits, tok_out, tok_stride, B, c.vocab, st));
+  if (tok_out != nullptr) {
+    if (sample_pos >= 0)
+      VCL_TRY(launch_sample(h->logits, c.vocab, B, c.vocab, h->d_sample, SampleParams{}, sample_pos, pos_dev, tok_out,
+                            tok_stride, st));
+    else
+      VCL_TRY(launch_argmax(h->logits, tok_out, tok_stride, B, c.vocab, st));
+  }
   return 0;
 }
 
@@ -677,19 +691,23 @@ int llm_decode_step(vcl_handle* h, const StepIo& io, int B, int pos, cudaStream_
       VCL_TRY(gemm(h->d_act, F, w.wd, F, h->d_h, D, nullptr, h->d_h, D, B, D, F, ACT_NONE, st));
     }
   }
-  VCL_TRY(lm_head_argmax(h, h->d_h, D, B, io.logits_out, io.tok_out, io.out_stride, st, io.partials_out));
+  VCL_REQUIRE(!(io.sample && io.partials_out), "a sampled step has no partial arg-max hand-off");
+  VCL_TRY(lm_head_argmax(h, h->d_h, D, B, io.logits_out, io.tok_out, io.out_stride, st, io.partials_out,
+                         io.sample ? pos + 1 : -1, pd));
   return 0;
 }
 
 // Steps 1 .. n_new-1 of a greedy loop over the token scratch tk [B][n_new] (tk[:, 0] is given).
 // On the ring-kernel path no arg-max / embedding kernel runs between two steps: the logits kernel
 // leaves per-CTA partials, the next step's first q|k|v kernel reduces them, records the token and
-// gathers its embedding row.
-int decode_steps(vcl_handle* h, int32_t* tk, int B, int S, int n_new, const int* pos_dev, cudaStream_t st) {
-  const bool hand_off = tc_batch(h, B) && h->cfg.llm_layers > 0;
+// gathers its embedding row. A sampled loop (mode MODE_SAMPLED) has no hand-off: every step writes
+// full logits, the sampler writes tk[:, i] and the next step gathers the row from there.
+int decode_steps(vcl_handle* h, int32_t* tk, int B, int S, int n_new, const int* pos_dev, int mode, cudaStream_t st) {
+  const bool hand_off = mode == MODE_GREEDY && tc_batch(h, B) && h->cfg.llm_layers > 0;
   for (int i = 1; i < n_new; ++i) {
     StepIo io;
     io.pos_dev = pos_dev;
+    io.sample = mode == MODE_SAMPLED;
     if (hand_off && i > 1) {
       io.tok_from_partials = true; io.tok_store = tk + (i - 1); io.store_stride = n_new;
     } else {
@@ -777,24 +795,38 @@ int vcl_llm_decode_step(vcl_handle* h, const int32_t* tok_in, int B, int pos, fl
   return llm_decode_step(h, io, B, pos, as_stream(stream));
 }
 
-int vcl_llm_decode_loop(vcl_handle* h, const int32_t* first_tok, int B, int S, int n_new,
-                        int32_t* out_tokens, void* stream) {
+}  // extern "C"
+
+namespace {
+
+int check_sampling(const vcl_sampling* sp) {
+  VCL_REQUIRE(sp != nullptr, "sampling parameters are required");
+  VCL_REQUIRE(!isnan(sp->temperature), "sampling temperature is NaN");
+  return 0;
+}
+
+SampleParams sample_params(const vcl_sampling* sp) { return SampleParams{sp->temperature, sp->top_k, sp->seed}; }
+
+// vcl_llm_decode_loop (MODE_GREEDY) and vcl_llm_decode_loop_sampled (MODE_SAMPLED: h->d_sample holds the
+// parameters, written on the stream before this is called)
+int decode_loop(vcl_handle* h, const int32_t* first_tok, int B, int S, int n_new, int mode, int32_t* out_tokens,
+                cudaStream_t st) {
   VCL_REQUIRE(h && first_tok && out_tokens, "vcl_llm_decode_loop: null argument");
   VCL_REQUIRE(h->llm_loaded, "LLM weights are not loaded");
   VCL_REQUIRE(B > 0 && B <= h->cfg.max_batch, "B=%d outside 1..%d", B, h->cfg.max_batch);
   VCL_REQUIRE(n_new >= 1 && S + n_new <= h->cfg.max_seq + 1, "S + n_new = %d exceeds max_seq %d", S + n_new,
               h->cfg.max_seq);
-  cudaStream_t st = as_stream(stream);
   int32_t* tk = h->tokens;  // [B, n_new] row-major scratch
   if (first_tok != tk)
     VCL_CUDA_OK(cudaMemcpy2DAsync(tk, (size_t)n_new * sizeof(int32_t), first_tok, sizeof(int32_t),
                                   sizeof(int32_t), B, cudaMemcpyDeviceToDevice, st));
   if (n_new > 1) {
-    // One graph per (B, n_new): the prompt length S reaches the kernels through h->d_pos, so a new
-    // prompt length replays the same graph. Bounded LRU cache (an entry holds thousands of nodes).
+    // One graph per (B, n_new, mode): the prompt length S reaches the kernels through h->d_pos (and the
+    // sampling parameters through h->d_sample), so a new prompt length replays the same graph. Bounded
+    // LRU cache (an entry holds thousands of nodes).
     GraphEntry* ge = nullptr;
     for (auto& g : h->graphs)
-      if (g.B == B && g.n_new == n_new && g.S == -1) ge = &g;
+      if (g.B == B && g.n_new == n_new && g.S == -1 && g.mode == mode) ge = &g;
     const bool can_capture = (st != nullptr) && (st != cudaStreamLegacy);
     if (ge == nullptr && can_capture) {
       if (h->graphs.size() >= MAX_DECODE_GRAPHS) {
@@ -806,7 +838,7 @@ int vcl_llm_decode_loop(vcl_handle* h, const int32_t* first_tok, int B, int S, i
       }
       const long long before = launch_count();
       VCL_CUDA_OK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-      const int rc = decode_steps(h, tk, B, S, n_new, h->d_pos, st);
+      const int rc = decode_steps(h, tk, B, S, n_new, h->d_pos, mode, st);
       cudaGraph_t graph = nullptr;
       cudaError_t e = cudaStreamEndCapture(st, &graph);
       const long long nodes = launch_count() - before;
@@ -826,7 +858,7 @@ int vcl_llm_decode_loop(vcl_handle* h, const int32_t* first_tok, int B, int S, i
         set_last_error("decode graph instantiate failed: %s", cudaGetErrorString(e));
         return -2;
       }
-      h->graphs.push_back({B, -1, n_new, exec, nodes, 0});
+      h->graphs.push_back({B, -1, n_new, mode, exec, nodes, 0});
       ge = &h->graphs.back();
     }
     if (ge != nullptr) {
@@ -835,11 +867,29 @@ int vcl_llm_decode_loop(vcl_handle* h, const int32_t* first_tok, int B, int S, i
       VCL_CUDA_OK(cudaGraphLaunch(ge->exec, st));
       count_launches(ge->kernels);
     } else {
-      VCL_TRY(decode_steps(h, tk, B, S, n_new, nullptr, st));
+      VCL_TRY(decode_steps(h, tk, B, S, n_new, nullptr, mode, st));
     }
   }
   VCL_CUDA_OK(cudaMemcpyAsync(out_tokens, tk, (size_t)B * n_new * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
   return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int vcl_llm_decode_loop(vcl_handle* h, const int32_t* first_tok, int B, int S, int n_new,
+                        int32_t* out_tokens, void* stream) {
+  return decode_loop(h, first_tok, B, S, n_new, MODE_GREEDY, out_tokens, as_stream(stream));
+}
+
+int vcl_llm_decode_loop_sampled(vcl_handle* h, const int32_t* first_tok, int B, int S, int n_new,
+                                const vcl_sampling* sampling, int32_t* out_tokens, void* stream) {
+  VCL_REQUIRE(h != nullptr, "vcl_llm_decode_loop_sampled: null handle");
+  VCL_TRY(check_sampling(sampling));
+  cudaStream_t st = as_stream(stream);
+  VCL_TRY(launch_set_sample_params(h->d_sample, sample_params(sampling), st));
+  return decode_loop(h, first_tok, B, S, n_new, MODE_SAMPLED, out_tokens, st);
 }
 
 int vcl_llm_generate(vcl_handle* h, const int64_t* ids, const void* video_feats,
@@ -854,7 +904,33 @@ int vcl_llm_generate(vcl_handle* h, const int64_t* ids, const void* video_feats,
   return vcl_llm_decode_loop(h, h->tokens, B, S, n_new, out_tokens, stream);
 }
 
+int vcl_llm_generate_sampled(vcl_handle* h, const int64_t* ids, const void* video_feats, const int32_t* vid_start,
+                             int B, int S, int n_new, const vcl_sampling* sampling, int32_t* out_tokens,
+                             void* stream) {
+  VCL_REQUIRE(h && out_tokens, "vcl_llm_generate_sampled: null argument");
+  VCL_TRY(check_sampling(sampling));
+  VCL_REQUIRE(n_new >= 1 && S + n_new <= h->cfg.max_seq + 1, "S + n_new = %d exceeds max_seq %d", S + n_new,
+              h->cfg.max_seq);
+  cudaStream_t st = as_stream(stream);
+  VCL_TRY(launch_set_sample_params(h->d_sample, sample_params(sampling), st));
+  // the prefill leaves its last-position logits in h->logits; the first new token takes position S
+  VCL_TRY(llm_prefill(h, ids, video_feats, vid_start, B, S, h->cfg.llm_layers, nullptr, h->logits, nullptr, 1, st));
+  VCL_TRY(launch_sample(h->logits, h->cfg.vocab, B, h->cfg.vocab, h->d_sample, SampleParams{}, S, nullptr, h->tokens,
+                        n_new, st));
+  return decode_loop(h, h->tokens, B, S, n_new, MODE_SAMPLED, out_tokens, st);
+}
+
 long long vcl_launch_count(void) { return launch_count(); }
+
+int vcl_op_sample(const float* logits, int64_t ld, int B, int V, const vcl_sampling* sampling, int pos,
+                  int32_t* tok_out, void* stream) {
+  VCL_REQUIRE(logits && tok_out, "vcl_op_sample: null argument");
+  VCL_TRY(check_sampling(sampling));
+  VCL_REQUIRE(B >= 0 && pos >= 0, "vcl_op_sample: B=%d pos=%d", B, pos);
+  if (check_device() != 0) return -2;
+  return launch_sample(logits, ld, B, V, nullptr, sample_params(sampling), pos, nullptr, tok_out, 1,
+                       as_stream(stream));
+}
 
 // ---- single-operator entry points ----
 int vcl_op_gemm(const void* A, int64_t lda, const void* W, int64_t ldw, void* C, int64_t ldc,

@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int64, c_void_p
+from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int64, c_uint64, c_void_p
 
 import torch
 
@@ -42,6 +42,15 @@ class vcl_tensor(Structure):
     _fields_ = [("name", c_char_p), ("data", c_void_p), ("ndim", c_int32), ("shape", c_int64 * 4)]
 
 
+class vcl_sampling(Structure):
+    _fields_ = [("temperature", c_float), ("top_k", c_int32), ("seed", c_uint64)]
+
+
+def sampling(temperature: float, top_k, seed: int) -> vcl_sampling:
+    """The vcl_sampling struct (include/vcl.h); top_k None or 0 means no top-k filter."""
+    return vcl_sampling(float(temperature), int(top_k or 0), int(seed) & (2 ** 64 - 1))
+
+
 # name -> (restype, argtypes); mirrors include/vcl.h one to one
 _SIGNATURES = {
     "vcl_version": (c_int, []),
@@ -62,6 +71,11 @@ _SIGNATURES = {
     "vcl_llm_generate": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p,
                                  c_void_p]),
     "vcl_llm_decode_loop": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "vcl_llm_generate_sampled": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                                         POINTER(vcl_sampling), c_void_p, c_void_p]),
+    "vcl_llm_decode_loop_sampled": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, POINTER(vcl_sampling), c_void_p,
+                                            c_void_p]),
+    "vcl_op_sample": (c_int, [c_void_p, c_int64, c_int, c_int, POINTER(vcl_sampling), c_int, c_void_p, c_void_p]),
     "vcl_launch_count": (ctypes.c_longlong, []),
     "vcl_op_gemm": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p,
                             c_int64, c_int, c_int, c_int, c_int, c_int, c_void_p]),
@@ -180,6 +194,18 @@ def op_gemv(x, w, res=None, norm_w=None, eps=0.0):
     out = torch.empty(B, N, dtype=torch.bfloat16, device=x.device)
     check(lib().vcl_op_gemv(ptr(x), ptr(w), ptr(out), ptr(res), ptr(norm_w), eps, B, N, K, cur_stream()))
     return out
+
+
+def op_sample(logits, temperature, top_k, seed, pos):
+    """[B, V] fp32 logits (row stride may exceed V) -> [B] int32 tokens for sequence position `pos`
+    (the contract of vcl_sampling)."""
+    B, V = logits.shape
+    assert logits.is_cuda and logits.dtype == torch.float32 and logits.stride(1) == 1
+    tok = torch.empty(B, dtype=torch.int32, device=logits.device)
+    sp = sampling(temperature, top_k, seed)
+    check(lib().vcl_op_sample(c_void_p(logits.data_ptr()), logits.stride(0), B, V, ctypes.byref(sp), int(pos),
+                              ptr(tok), cur_stream()))
+    return tok
 
 
 # ---------------------------------------------------------------------------------------------
@@ -343,4 +369,24 @@ class Engine:
             vf = video_feats.to(torch.bfloat16).contiguous()
         check(lib().vcl_llm_generate(self._h, ptr(ids.contiguous()), ptr(vf), ptr(vid_start.contiguous()), B, S,
                                      n_new, ptr(out), cur_stream()))
+        return out
+
+    def generate_sampled(self, ids, video_feats, vid_start, n_new, temperature, top_k, seed):
+        B, S = ids.shape
+        out = torch.empty(B, n_new, dtype=torch.int32, device=ids.device)
+        vf = None
+        if video_feats is not None:
+            vf = video_feats.to(torch.bfloat16).contiguous()
+        sp = sampling(temperature, top_k, seed)
+        check(lib().vcl_llm_generate_sampled(self._h, ptr(ids.contiguous()), ptr(vf), ptr(vid_start.contiguous()), B,
+                                             S, n_new, ctypes.byref(sp), ptr(out), cur_stream()))
+        return out
+
+    def decode_loop_sampled(self, first_tok, S, n_new, temperature, top_k, seed, out=None):
+        B = first_tok.shape[0]
+        if out is None:
+            out = torch.empty(B, n_new, dtype=torch.int32, device=first_tok.device)
+        sp = sampling(temperature, top_k, seed)
+        check(lib().vcl_llm_decode_loop_sampled(self._h, ptr(first_tok.contiguous()), B, S, n_new, ctypes.byref(sp),
+                                                ptr(out), cur_stream()))
         return out

@@ -37,6 +37,12 @@ from ..constants import (DEFAULT_VID_END_TOKEN, DEFAULT_VID_START_TOKEN,  # noqa
 from .multimodal_projector.builder import build_vision_projector  # noqa: E402
 
 
+def _host_sampling() -> bool:
+    """VCL_HOST_SAMPLING=1: sampling and stopping criteria take one C-ABI step per token with host-side
+    sampling (torch.topk / softmax / multinomial) instead of the device sampler and chunked decode loops."""
+    return os.environ.get("VCL_HOST_SAMPLING") == "1"
+
+
 class VisionConfig:
     def __init__(self, frame_size=224, patch_size=14, hidden_size=1024):
         self.frame_size = frame_size
@@ -425,11 +431,13 @@ class VideoChatGPTLlamaForCausalLM:
         """Returns [B, S+n] int64 INCLUDING the prompt, like HF generate (inference.py:105-120), and
         like HF it stops at EOS (config.eos_token_id unless eos_token_id is given; None disables it):
         finished rows are padded, the call returns when every row has finished.
-        Greedy decoding without stopping criteria runs on the device: prefill + CUDA-graph decode
-        loops of 32 tokens with one host-side EOS check per loop (a single loop of exactly
-        max_new_tokens when EOS is disabled). Sampling (temperature, top-k 50 as HF defaults) or
-        stopping criteria take one C-ABI step per token with the host-side check the reference also
-        performs every step."""
+        Everything runs on the device: prefill + CUDA-graph decode loops of 32 tokens with one host-side
+        check per loop (a single loop of exactly max_new_tokens for greedy decoding without EOS or
+        stopping criteria). Sampling (temperature, top-k 50 as HF defaults) uses the device sampler
+        (include/vcl.h, vcl_sampling) with a seed drawn from torch's default CPU generator, so
+        torch.manual_seed makes runs reproducible. Stopping criteria are called after each loop, exactly
+        as a per-token loop would call them (_replay). VCL_HOST_SAMPLING=1 in the environment keeps the
+        per-token C-ABI step with host-side sampling and checks (_stepwise) for sampling and criteria."""
         eng = self._ensure_engine(need_llm=True)
         ids = input_ids.cuda().to(torch.int64)
         B, S = ids.shape
@@ -441,11 +449,19 @@ class VideoChatGPTLlamaForCausalLM:
         if n <= 0:
             raise ValueError(f"prompt length {S} leaves no room in max_seq {self._max_seq}")
         eos, pad = self._eos_pad(eos_token_id, pad_token_id)
-        if do_sample or stopping_criteria:
+        if (do_sample or stopping_criteria) and _host_sampling():
             _, logits, _ = eng.prefill(ids, feats, vs, want_logits=True, want_token=False)
             self._pos = S
             self._last_out = self._stepwise(eng, ids, logits, n, do_sample, temperature, stopping_criteria, eos, pad,
                                             top_k)
+            return self._last_out
+        if (do_sample and temperature > 0) or stopping_criteria:
+            sp = self._sampling(do_sample, temperature, top_k)
+            if sp is None:
+                first_chunk = lambda c: eng.generate(ids, feats, vs, c)
+            else:
+                first_chunk = lambda c: eng.generate_sampled(ids, feats, vs, c, *sp)
+            self._last_out = self._device_decode(eng, ids, first_chunk, n, sp, stopping_criteria, eos, pad)
             return self._last_out
         if eos is None:
             new = eng.generate(ids, feats, vs, n).to(torch.int64)
@@ -496,13 +512,85 @@ class VideoChatGPTLlamaForCausalLM:
         if n <= 0:
             raise ValueError(f"context length {ctx.shape[1]} leaves no room in max_seq {self._max_seq}")
         eos, pad = self._eos_pad(eos_token_id, pad_token_id)
-        _, logits, _ = eng.prefill_append(tail, start, want_logits=True, want_token=False)
-        self._pos = ctx.shape[1]
-        self._last_out = self._stepwise(eng, ctx, logits, n, do_sample, temperature, stopping_criteria, eos, pad, top_k)
+        if _host_sampling():
+            _, logits, _ = eng.prefill_append(tail, start, want_logits=True, want_token=False)
+            self._pos = ctx.shape[1]
+            self._last_out = self._stepwise(eng, ctx, logits, n, do_sample, temperature, stopping_criteria, eos, pad,
+                                            top_k)
+            return self._last_out
+        sp = self._sampling(do_sample, temperature, top_k)
+        P0 = ctx.shape[1]                                       # position of the first new token
+        if sp is None:
+            _, _, first = eng.prefill_append(tail, start, want_token=True)
+            first_chunk = lambda c: eng.decode_loop(first, P0, c)
+        else:
+            _, logits, _ = eng.prefill_append(tail, start, want_logits=True, want_token=False)
+            first = vn.op_sample(logits, *sp, pos=P0)
+            first_chunk = lambda c: eng.decode_loop_sampled(first, P0, c, *sp)
+        self._last_out = self._device_decode(eng, ctx, first_chunk, n, sp, stopping_criteria, eos, pad)
         return self._last_out
 
+    @staticmethod
+    def _sampling(do_sample, temperature, top_k):
+        """(temperature, top_k, seed) for the device sampler, None for greedy decoding. The seed comes from
+        torch's default CPU generator, one draw per call."""
+        if not (do_sample and temperature > 0):
+            return None
+        seed = int(torch.randint(0, 2 ** 63 - 1, (1,)))
+        return float(temperature), int(top_k or 0), seed
+
+    def _device_decode(self, eng, out, first_chunk, n, sp, stopping_criteria, eos, pad):
+        """Up to n new tokens after `out` [B, P0] in device loops of _GREEDY_CHUNK tokens; first_chunk(c) gives
+        the first c tokens ([B, c] int32, token 0 at position P0), later loops continue from the last token.
+        After each loop _replay makes the calls _stepwise would have made, in the same order, and cuts `out`
+        where _stepwise would have stopped. Tokens computed past that point stay in the KV cache as dead rows:
+        decode attention reads only pos + 1 keys and the next prefill (generate_continue) overwrites them."""
+        P0 = out.shape[1]
+        unfinished = torch.ones(out.shape[0], dtype=torch.bool)
+        new = first_chunk(min(n, self._GREEDY_CHUNK))
+        k = 0
+        while True:
+            out, unfinished, stopped = self._replay(out, new, unfinished, stopping_criteria, eos, pad)
+            k += new.shape[1]
+            if stopped or k >= n:
+                break
+            m = min(self._GREEDY_CHUNK, n - k)
+            last = new[:, -1].to(torch.int32).contiguous()
+            more = (eng.decode_loop(last, P0 + k - 1, m + 1) if sp is None
+                    else eng.decode_loop_sampled(last, P0 + k - 1, m + 1, *sp))
+            new = more[:, 1:]
+        self._pos = out.shape[1] - 1
+        return out
+
+    @staticmethod
+    def _replay(out, new, unfinished, stopping_criteria, eos, pad):
+        """_stepwise's per-token bookkeeping over the device tokens `new` [B, c]: append each token (pad if
+        its row has finished), update `unfinished`, stop when no row is left, else call every criterion on
+        the prefix and stop at the first True. Returns (out, unfinished, stopped)."""
+        new_h = new.to(device="cpu", dtype=torch.int64)
+        cols = []
+        stopped = False
+        for j in range(new_h.shape[1]):
+            nxt = new_h[:, j]
+            if eos is not None:
+                nxt = torch.where(unfinished, nxt, torch.full_like(nxt, pad))
+            cols.append(nxt)
+            if stopping_criteria:
+                out = torch.cat([out, nxt[:, None].to(out.device)], dim=1)   # the prefix the criteria see
+            if eos is not None:
+                unfinished = unfinished & (nxt != eos)
+                if not bool(unfinished.any()):
+                    stopped = True
+                    break
+            if stopping_criteria and any(c(out, None) for c in stopping_criteria):
+                stopped = True
+                break
+        if not stopping_criteria:
+            out = torch.cat([out, torch.stack(cols, dim=1).to(out.device)], dim=1)
+        return out, unfinished, stopped
+
     def _stepwise(self, eng, out, logits, n, do_sample, temperature, stopping_criteria, eos, pad, top_k=50):
-        """One token per C-ABI call. After the loop the cache holds every returned token but the last
+        """One token per C-ABI call (VCL_HOST_SAMPLING=1). After the loop the cache holds every returned token but the last
         (self._pos = out.shape[1] - 1), the state generate_continue starts from."""
         unfinished = torch.ones(out.shape[0], dtype=torch.bool, device=out.device)
         for step in range(n):
